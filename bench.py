@@ -54,7 +54,26 @@ def parse():
     ap.add_argument("--passes", type=int, default=16, help="passes over the batch per step (timed region >= 0.5 s at the default K)")
     ap.add_argument("--no-extra", action="store_true", help="headline only (profiling runs)")
     ap.add_argument("--only", default="", help="comma-separated subset of the secondary workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the headline encode produced in the last one "
+                    "(a fixed sample of the DXT1 blocks of every frame of rank 0) to DIR/*.npy")
     return ap.parse_args()
+
+
+DUMP_BYTES = 48 << 20  # the dump stays well below 64 MB whatever the batch size
+
+
+def dump_dxt1(outs, out_dir):
+    """DIR/dxt1_blocks.npy: float64 (frames, blocks, 2), the two 32-bit words (colours, indices) of the same seeded sample of block
+    positions in every frame; DIR/dxt1_block_index.npy: those positions (row-major 4x4 blocks).  The integers are exact in float64."""
+    import numpy as np
+    import torch
+    n_frames, n_blocks = outs.shape[0], outs.shape[1] // 8
+    n = min(n_blocks, DUMP_BYTES // (16 * n_frames + 8))  # 16 bytes per block and frame, 8 per position
+    idx = np.sort(np.random.default_rng(0).choice(n_blocks, size=n, replace=False))
+    words = outs.view(torch.int32).reshape(n_frames, n_blocks, 2)[:, torch.from_numpy(idx).to(outs.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "dxt1_blocks.npy"), (words.cpu().numpy().astype(np.int64) & 0xFFFFFFFF).astype(np.float64))
+    np.save(os.path.join(out_dir, "dxt1_block_index.npy"), idx.astype(np.float64))
 
 
 def measured_peaks():
@@ -626,6 +645,8 @@ def main():
     clk = clocks.stop() if rank == 0 else None
     ms_max = max_over_ranks(ms)
     fps = world * B * P * K / (ms_max * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_dxt1(outs, args.dump_outputs)
 
     # ---- end to end through the reference-facing plugin: compress_init("cuda_dxt:DXT1") with pinned HOST frames -------------------------------
     hosts = [host_copy(ctx, frames[i]) for i in range(6)]

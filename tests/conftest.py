@@ -17,12 +17,3 @@ def pytest_configure(config):
 def orc():
     import util
     return util.oracle()
-
-
-@pytest.fixture(scope="session")
-def ref_cpu():
-    import util
-    lib = util.ref_cpu()
-    if lib is None:
-        pytest.skip("oracle/_ref/libugref.so not built (reference tree absent)")
-    return lib

@@ -1,6 +1,6 @@
 """src/utils/cuda_pix_conv.cu of the reference (SURVEY.md section 8f rank 4): cuda_RGB_to_RGBA, cuda_RGBA_to_RGB, cuda_UYVY_to_RGBA,
-cuda_RGBA_to_UYVY with the reference's C++ names.  GPU: libugb200 == the UNMODIFIED reference file built for sm_100a (oracle/_ref) == the CPU
-restatement, byte for byte."""
+cuda_RGBA_to_UYVY with the reference's C++ names.  GPU: libugb200 == the UNMODIFIED reference file built for sm_100a (oracle/_ref; its outputs
+recorded in tests/golden/reference_cuda_pix_conv.json) == the CPU restatement, byte for byte."""
 import ctypes
 import os
 
@@ -27,8 +27,6 @@ def test_gpu_equals_reference_kernels_and_restatement(orc, name):
     import torch
     from ultragrid_b200 import _lib
     lib = ctypes.CDLL(_lib.LIB_PATH)
-    ref_path = os.path.join(util.ORACLE_DIR, "_ref", "libcuda_pix_conv_ref.so")
-    ref = ctypes.CDLL(ref_path) if os.path.exists(ref_path) else None
     sym, kind, bi, bo = NAMES[name]
     orc.orc_cuda_pix_conv.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int, ctypes.c_int]
     orc.orc_cuda_pix_conv.restype = None
@@ -39,15 +37,16 @@ def test_gpu_equals_reference_kernels_and_restatement(orc, name):
         want = np.full(dp * h, 0xCD, np.uint8)
         orc.orc_cuda_pix_conv(kind, want.ctypes.data, dp, src.ctypes.data, sp, w, h)
         d_src = torch.from_numpy(src).cuda()
-        outs = []
-        for L in (lib, ref):
-            if L is None:
-                continue
+
+        def run(L):
             fn = getattr(L, sym)
             fn.argtypes, fn.restype = ARGS, None
             d_dst = torch.full((dp * h,), 0xCD, dtype=torch.uint8, device="cuda")
             fn(d_dst.data_ptr(), dp, d_src.data_ptr(), sp, w, h, None)
             torch.cuda.synchronize()
-            outs.append(d_dst.cpu().numpy())
-        for o in outs:
-            assert np.array_equal(o, want), (name, w, h, pad, np.flatnonzero(o != want)[:8])
+            return d_dst.cpu().numpy()
+        o = run(lib)
+        assert np.array_equal(o, want), (name, w, h, pad, np.flatnonzero(o != want)[:8])
+        theirs = util.reference("cuda_pix_conv", f"{name}/{w}x{h}+{pad}",
+                                lambda: util.digest(run(ctypes.CDLL(os.path.join(util.ORACLE_DIR, "_ref", "libcuda_pix_conv_ref.so")))))
+        assert util.digest(want) == theirs, (name, w, h, pad)

@@ -28,18 +28,16 @@ def test_library_exports_the_reference_cxx_symbols():
     assert hasattr(lib, POST) and hasattr(lib, PRE)
 
 
-def libs():
+def entry_points(path):
+    """(postprocess_rg48_to_r12l, preprocess_r12l_to_rg48) of libugb200, or of the reference build when path is given"""
     from ultragrid_b200 import _lib
-    lib = ctypes.CDLL(_lib.LIB_PATH)
-    ref_path = os.path.join(util.ORACLE_DIR, "_ref", "libcuda_wrapper_kernels_ref.so")
-    ref = ctypes.CDLL(ref_path) if os.path.exists(ref_path) else None
-    out = []
-    for L in (lib, ref):
-        if L is not None:
-            post, pre = getattr(L, POST), getattr(L, PRE)
-            post.argtypes, post.restype, pre.argtypes, pre.restype = POST_ARGS, I, PRE_ARGS, I
-            out.append((post, pre))
-    return out
+    L = ctypes.CDLL(path or _lib.LIB_PATH)
+    post, pre = getattr(L, POST), getattr(L, PRE)
+    post.argtypes, post.restype, pre.argtypes, pre.restype = POST_ARGS, I, PRE_ARGS, I
+    return post, pre
+
+
+REF = os.path.join(util.ORACLE_DIR, "_ref", "libcuda_wrapper_kernels_ref.so")  # its outputs are recorded in tests/golden/reference_cuda_wrapper_kernels.json
 
 
 SIZES = [(8, 1), (16, 3), (64, 2), (256, 5), (1920, 8), (7680, 4), (4, 2), (9, 3), (30, 2), (1000, 3), (1921, 2), (255, 4)]
@@ -52,19 +50,21 @@ def test_rg48_to_r12l_equals_reference_kernel(orc, w, h):
     nb = (w + 7) // 8
     src = util.rng_bytes(w * 6 * h, 700 + w)
     d_src = torch.from_numpy(src).cuda()
-    outs = []
-    for post, _ in libs():
+
+    def run(path):
+        post, _ = entry_points(path)
         d_dst = torch.full((nb * 36 * h,), 0xCD, dtype=torch.uint8, device="cuda")
         assert post(None, None, 0, w, h, None, 3, d_src.data_ptr(), src.size, None, 0, d_dst.data_ptr(), d_dst.numel(), None) == 0
         torch.cuda.synchronize()
-        outs.append(d_dst.cpu().numpy().reshape(h, nb * 36))
+        return d_dst.cpu().numpy().reshape(h, nb * 36)
+    outs = [run(None)]
     # the whole groups are vc_copylineRG48toR12L of the pinned oracle
     want = util.convert_cpu(orc, "orc_convert", RG48, R12L, src, w, h, src_pitch=w * 6, dst_pitch=nb * 36, dst_len=nb * 36).reshape(h, nb * 36)
     full = w // 8 * 36
     defined = full + (w % 8) * 36 // 8  # bytes of the last group that depend only on samples inside the row (4.5 bytes per pixel, rounded down)
-    for o in outs:
-        assert np.array_equal(o[:, :full], want[:, :full])
-        assert np.array_equal(o[:, :defined], outs[0][:, :defined])
+    assert np.array_equal(outs[0][:, :full], want[:, :full])
+    # the reference kernel: its defined bytes equal ours (and so the oracle's whole groups)
+    assert util.digest(outs[0][:, :defined]) == util.reference("cuda_wrapper_kernels", f"rg48_to_r12l/{w}x{h}", lambda: util.digest(run(REF)[:, :defined]))
     if w % 8:  # the partial group is written (the CPU line converter stops before it): its defined bytes are the packed samples
         s16 = src.view(np.uint16).reshape(h, w * 3)[:, w // 8 * 24:] >> 4
         bits = np.zeros((h, 36), np.uint8)
@@ -83,13 +83,16 @@ def test_r12l_to_rg48_equals_reference_kernel(orc, w, h):
     nb = (w + 7) // 8
     src = util.rng_bytes(nb * 36 * h, 800 + w)
     d_src = torch.from_numpy(src).cuda()
-    outs = []
-    for _, pre in libs():
+
+    def run(path):
+        _, pre = entry_points(path)
         d_dst = torch.full((w * 6 * h + 64,), 0xCD, dtype=torch.uint8, device="cuda")
         assert pre(None, None, 0, w, h, None, 3, d_src.data_ptr(), src.size, d_dst.data_ptr(), w * 6 * h, None) == 0
         torch.cuda.synchronize()
-        outs.append(d_dst.cpu().numpy())
+        return d_dst.cpu().numpy()
+    o = run(None)
     want = util.convert_cpu(orc, "orc_convert", R12L, RG48, src, w, h, src_pitch=nb * 36, dst_pitch=w * 6, dst_len=w * 6)
-    for o in outs:
-        assert np.array_equal(o[:w * 6 * h], want)
-        assert np.all(o[w * 6 * h:] == 0xCD)  # exactly size_x * 6 bytes per row, nothing behind the frame
+    assert np.array_equal(o[:w * 6 * h], want)
+    assert np.all(o[w * 6 * h:] == 0xCD)  # exactly size_x * 6 bytes per row, nothing behind the frame
+    # the reference kernel wrote the same bytes, and nothing else
+    assert util.digest(o) == util.reference("cuda_wrapper_kernels", f"r12l_to_rg48/{w}x{h}", lambda: util.digest(run(REF)))

@@ -16,12 +16,9 @@ class Coeffs(ctypes.Structure):
     _fields_ = [(n, _i) for n in ("y_r", "y_g", "y_b", "cb_r", "cb_g", "cb_b", "cr_r", "cr_g", "cr_b")]
 
 
-def coeffs(ref_cpu, depth):
+def coeffs(depth):
     """get_color_coeffs(CS_DFL, depth) of the UNMODIFIED src/color_space.c"""
-    out = (_i * 14)()
-    ref_cpu.ref_get_color_coeffs.argtypes = [_i, _i, _vp]
-    ref_cpu.ref_get_color_coeffs(0, depth, out)
-    return Coeffs(*list(out)[:9])
+    return Coeffs(*util.ref_color_coeffs(0, depth)[:9])
 
 
 def planes_for(shapes, fill=0xA5):
@@ -31,7 +28,7 @@ def planes_for(shapes, fill=0xA5):
     return bufs, p, ls
 
 
-def lavc_cpu(orc, ref_cpu, in_codec, fmt, src, w, h, pad=0):
+def lavc_cpu(orc, in_codec, fmt, src, w, h, pad=0):
     from ultragrid_b200 import api
     shapes = api.av_plane_shapes(fmt, w, h, pad)
     bufs, p, ls = planes_for(shapes)
@@ -44,7 +41,7 @@ def lavc_cpu(orc, ref_cpu, in_codec, fmt, src, w, h, pad=0):
     else:
         depth = 8 if fmt == "YUV444P" else int(fmt[7:9])
         kind = {R10k: 0, RG48: 1, R12L: 2, RGB: 3}[in_codec]
-        orc.orc_lavc_rgb(kind, depth, 1 if "422" in fmt else 0, ctypes.byref(coeffs(ref_cpu, depth)), src.ctypes.data, w, h, p, ls)
+        orc.orc_lavc_rgb(kind, depth, 1 if "422" in fmt else 0, ctypes.byref(coeffs(depth)), src.ctypes.data, w, h, p, ls)
     return bufs, shapes
 
 
@@ -71,33 +68,40 @@ def test_support_table_and_hook_refusals():
     assert not L.ugb200_get_av_to_uv_conversion(api.AV_PIXFMT["NV12"], UYVY)
 
 
-def test_restatement_v210_identities_through_reference_functions(orc, ref_cpu):
+def test_restatement_v210_identities_through_reference_functions(orc):
     """v210 -> yuv422p10le -> (UNMODIFIED yuv422p10le_to_v210, from_planar.c:295-333) == the v210 frame (30 valid bits per word), and
     v210 -> yuv420p10le == UNMODIFIED v210_to_p010le >> 6 (to_planar.c:64-155): the idea of test/ff_codec_conversions_test.cpp:346-401"""
     w, h = 96, 6
     src = util.v210_noise(w, h, 4)
-    bufs, shapes = lavc_cpu(orc, ref_cpu, V210, "YUV422P10LE", src, w, h)
-    back = np.zeros_like(src)
-    ref_cpu.ref_yuv422p10le_to_v210.argtypes = [_i, _i, _vp, ctypes.c_uint, _vp, _vp, _vp, ctypes.c_uint, ctypes.c_uint]
-    ref_cpu.ref_yuv422p10le_to_v210(w, h, back.ctypes.data, len(src) // h, bufs[0].ctypes.data, bufs[1].ctypes.data, bufs[2].ctypes.data, shapes[0][0], shapes[1][0])
-    assert np.array_equal(back, src)
+    bufs, shapes = lavc_cpu(orc, V210, "YUV422P10LE", src, w, h)
+
+    def back():  # the planes and what the reference packs them back into
+        ref = util.ref_cpu()
+        out = np.zeros_like(src)
+        ref.ref_yuv422p10le_to_v210.argtypes = [_i, _i, _vp, ctypes.c_uint, _vp, _vp, _vp, ctypes.c_uint, ctypes.c_uint]
+        ref.ref_yuv422p10le_to_v210(w, h, out.ctypes.data, len(src) // h, bufs[0].ctypes.data, bufs[1].ctypes.data, bufs[2].ctypes.data, shapes[0][0], shapes[1][0])
+        return {"planes": util.digest(*bufs), "v210": util.digest(out)}
+    want = util.reference("lavc", "yuv422p10le_to_v210", back)
+    assert util.digest(*bufs) == want["planes"] and want["v210"] == util.digest(src)
     # 4:2:0: luma and averaged chroma against the reference's P010 converter (samples there sit in the 10 MSBs, chroma interleaved)
-    bufs, shapes = lavc_cpu(orc, ref_cpu, V210, "YUV420P10LE", src, w, h)
-    y, c = np.zeros(w * 2 * h, np.uint8), np.zeros(w * h, np.uint8)
-    ref_cpu.ref_v210_to_p010le(w, h, y.ctypes.data, w * 2, c.ctypes.data, w * 2, src.ctypes.data)
-    assert np.array_equal(bufs[0].view(np.uint16), y.view(np.uint16) >> 6)
-    cc = (c.view(np.uint16) >> 6).reshape(h // 2, w)
-    assert np.array_equal(bufs[1].view(np.uint16).reshape(h // 2, -1), cc[:, 0::2])
-    assert np.array_equal(bufs[2].view(np.uint16).reshape(h // 2, -1), cc[:, 1::2])
+    bufs, shapes = lavc_cpu(orc, V210, "YUV420P10LE", src, w, h)
+
+    def p010():
+        y, c = np.zeros(w * 2 * h, np.uint8), np.zeros(w * h, np.uint8)
+        util.ref_cpu().ref_v210_to_p010le(w, h, y.ctypes.data, w * 2, c.ctypes.data, w * 2, src.ctypes.data)
+        cc = (c.view(np.uint16) >> 6).reshape(h // 2, w)
+        return [util.digest(y.view(np.uint16) >> 6), util.digest(cc[:, 0::2]), util.digest(cc[:, 1::2])]
+    want = util.reference("lavc", "v210_to_p010le", p010)
+    assert [util.digest(b.view(np.uint16)) for b in bufs] == want
 
 
-def test_restatement_rgb_matrix_against_reference_line_converters(orc, ref_cpu):
+def test_restatement_rgb_matrix_against_reference_line_converters(orc):
     """RG48 -> yuv444p16le uses the same Q14 matrix at depth 16 as the reference's vc_copylineRG48toY416 -style converters use: spot values by hand
     (coefficients from the unmodified color_space.c), limited-range offsets, and a white / black / primary sanity sweep"""
-    c = coeffs(ref_cpu, 16)
+    c = coeffs(16)
     src = np.array([[65535, 65535, 65535], [0, 0, 0], [65535, 0, 0], [0, 65535, 0], [0, 0, 65535], [12345, 23456, 34567]], np.uint16)
     w, h = len(src), 1
-    bufs, _ = lavc_cpu(orc, ref_cpu, RG48, "YUV444P16LE", src.view(np.uint8).reshape(-1), w, h)
+    bufs, _ = lavc_cpu(orc, RG48, "YUV444P16LE", src.view(np.uint8).reshape(-1), w, h)
     Y, CB, CR = (b.view(np.uint16)[:w].astype(np.int64) for b in bufs)
     for i, (r, g, b) in enumerate(src.astype(np.int64)):
         assert Y[i] == ((r * c.y_r + g * c.y_g + b * c.y_b) >> 14) + 4096
@@ -108,14 +112,14 @@ def test_restatement_rgb_matrix_against_reference_line_converters(orc, ref_cpu):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("inc,fmt", PAIRS)
-def test_gpu_to_lavc_equals_restatement(orc, ref_cpu, inc, fmt):
+def test_gpu_to_lavc_equals_restatement(orc, inc, fmt):
     import torch
     from ultragrid_b200 import api
     for k, (w, h, pad) in enumerate([(48, 4, 0), (96, 6, 32), (100, 5, 0), (8, 2, 0), (1920, 16, 64), (1922, 3, 10)]):
         if inc == V210 and fmt == "YUV420P10LE" and h % 2:
             h += 1
         src = source(orc, inc, w, h, 300 + k)
-        want, shapes = lavc_cpu(orc, ref_cpu, inc, fmt, src, w, h, pad)
+        want, shapes = lavc_cpu(orc, inc, fmt, src, w, h, pad)
         planes = [torch.full((ls * rows,), 0xA5, dtype=torch.uint8, device="cuda") for ls, rows in shapes]
         got = api.to_lavc(inc, fmt, torch.from_numpy(src).cuda(), w, h, planes=planes, pad=pad)
         for i, (g, wnt) in enumerate(zip(got, want)):
@@ -136,7 +140,7 @@ def test_gpu_delegated_conversions_equal_to_planar(orc):
 
 
 @pytest.mark.gpu
-def test_gpu_hook_shape_host_frame_in_device_planes_out(orc, ref_cpu):
+def test_gpu_hook_shape_host_frame_in_device_planes_out(orc):
     """to_lavc_vid_conv_cuda_init / to_lavc_vid_conv_cuda / _destroy (to_lavc_vid_conv_cuda.h:60-65): host frame in like the reference's hook"""
     import torch
     from ultragrid_b200 import _lib, api
@@ -146,7 +150,7 @@ def test_gpu_hook_shape_host_frame_in_device_planes_out(orc, ref_cpu):
     st = L.ugb200_to_lavc_vid_conv_init(UYVY, w, h, api.AV_PIXFMT["YUV444P"])  # the format the reference's hook names
     assert st
     p = ctypes.cast(L.ugb200_to_lavc_vid_conv(st, src.ctypes.data, 0), ctypes.POINTER(api.AvPlanes)).contents
-    want, shapes = lavc_cpu(orc, ref_cpu, UYVY, "YUV444P", src, w, h)
+    want, shapes = lavc_cpu(orc, UYVY, "YUV444P", src, w, h)
     for i in range(3):
         ls = p.linesize[i]
         host = np.zeros(ls * h, np.uint8)

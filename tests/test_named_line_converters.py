@@ -24,17 +24,15 @@ def run_cpu(lib, fn, fid, src, w, h, bi, bo, shifts, dst_len=None):
 
 @pytest.mark.parametrize("name", list(FUNCS))
 def test_restatement_equals_reference(orc, name):
-    ref = util.ref_cpu()
-    if ref is None or not hasattr(ref, "ref_copyline_named"):
-        pytest.skip("reference objects not built here (oracle/_ref)")
     fid, bi, bo = FUNCS[name]
-    for i, (w, h) in enumerate(SIZES):
-        src = util.rng_bytes(w * bi * h, 300 + i)
-        for shifts in SHIFTS:
-            for dl in (None, max(w * bo - 2, 0), max(w * bo - bo, 0)):
-                a = run_cpu(orc, "orc_copyline_named", fid, src, w, h, bi, bo, shifts, dl)
-                b = run_cpu(ref, "ref_copyline_named", fid, src, w, h, bi, bo, shifts, dl)
-                assert np.array_equal(a, b), (name, w, h, shifts, dl)
+    srcs = [util.rng_bytes(w * bi * h, 300 + i) for i, (w, h) in enumerate(SIZES)]
+
+    def run(lib, fn, src, w, h):  # every shift and dst_len of one size
+        return util.digest(*[run_cpu(lib, fn, fid, src, w, h, bi, bo, shifts, dl)
+                             for shifts in SHIFTS for dl in (None, max(w * bo - 2, 0), max(w * bo - bo, 0))])
+    want = util.reference("named_line_converters", name, lambda: [run(util.ref_cpu(), "ref_copyline_named", s, w, h) for s, (w, h) in zip(srcs, SIZES)])
+    for src, (w, h), d in zip(srcs, SIZES, want, strict=True):
+        assert run(orc, "orc_copyline_named", src, w, h) == d, (name, w, h)
 
 
 @pytest.mark.gpu

@@ -1,6 +1,6 @@
 """Pins the CPU restatement (oracle/*.c) before anything trusts it:
   1. known-answer checksums measured on the reference build (SURVEY.md section 6 / BASELINE.md section 2),
-  2. the unmodified reference objects (oracle/_ref/libugref.so) on ragged sizes, when built here,
+  2. the unmodified reference objects (oracle/_ref/libugref.so) on ragged sizes, as recorded in tests/golden/reference_*.json,
   3. committed golden vectors generated from the reference (tests/golden/make_golden.py),
   4. the colour-coefficient limits test of the reference (test/misc_test.c:46-87).
 """
@@ -41,13 +41,11 @@ def test_known_answer_checksums_8k(orc, inc, outc, chk):
 
 
 @pytest.mark.parametrize("depth", [0, 8, 10, 12, 16])
-def test_color_coeffs_vs_reference(orc, ref_cpu, depth):
+def test_color_coeffs_vs_reference(orc, depth):
     a = (ctypes.c_int * 14)()
-    b = (ctypes.c_int * 14)()
     for cs in (0, 1, 2):
         orc.orc_get_color_coeffs(cs, depth, a)
-        ref_cpu.ref_get_color_coeffs(cs, depth, b)
-        assert list(a) == list(b), (cs, depth)
+        assert list(a) == util.ref_color_coeffs(cs, depth), (cs, depth)
 
 
 def test_color_coeff_range(orc):
@@ -66,34 +64,42 @@ def test_color_coeff_range(orc):
 
 
 @pytest.mark.parametrize("inc,outc", PAIRS)
-def test_line_converters_vs_reference(orc, ref_cpu, inc, outc):
-    assert orc.orc_has_decoder(inc, outc) and ref_cpu.ref_has_decoder(inc, outc)
-    for i, (w, h) in enumerate([(1, 2), (2, 1), (6, 3), (16, 1), (17, 5), (47, 3), (48, 2), (50, 4), (127, 9), (130, 2), (256, 3)]):
-        assert orc.orc_vc_get_linesize(w, inc) == ref_cpu.ref_vc_get_linesize(w, inc)
+def test_line_converters_vs_reference(orc, inc, outc):
+    sizes = [(1, 2), (2, 1), (6, 3), (16, 1), (17, 5), (47, 3), (48, 2), (50, 4), (127, 9), (130, 2), (256, 3)]
+    cases = []  # per size: the source and the keyword arguments of every conversion of it
+    for i, (w, h) in enumerate(sizes):
         src = util.rng_bytes(orc.orc_vc_get_linesize(w, inc) * h, 1000 + i)
-        for shifts in ((0, 8, 16), (16, 8, 0), (8, 16, 24)):
-            a = util.convert_cpu(orc, "orc_convert", inc, outc, src, w, h, shifts=shifts)
-            b = util.convert_cpu(ref_cpu, "ref_convert", inc, outc, src, w, h, shifts=shifts)
-            assert np.array_equal(a, b), (w, h, shifts)
+        kws = [{"shifts": shifts} for shifts in ((0, 8, 16), (16, 8, 0), (8, 16, 24))]
         # a dst_len that is not a whole number of pixel groups (vc_get_size instead of linesize, ragged tails)
-        for dl in {orc.orc_vc_get_size(w, outc), max(orc.orc_vc_get_size(w, outc) - 4, 0) // 4 * 4}:
-            a = util.convert_cpu(orc, "orc_convert", inc, outc, src, w, h, dst_len=dl)
-            b = util.convert_cpu(ref_cpu, "ref_convert", inc, outc, src, w, h, dst_len=dl)
-            assert np.array_equal(a, b), (w, h, dl)
+        kws += [{"dst_len": dl} for dl in sorted({orc.orc_vc_get_size(w, outc), max(orc.orc_vc_get_size(w, outc) - 4, 0) // 4 * 4})]
+        cases.append((w, h, src, kws))
+
+    def run(lib, fn, w, h, src, kws):
+        return util.digest(*[util.convert_cpu(lib, fn, inc, outc, src, w, h, **kw) for kw in kws])
+
+    def theirs():
+        ref = util.ref_cpu()
+        return {"has_decoder": ref.ref_has_decoder(inc, outc), "linesize": [ref.ref_vc_get_linesize(w, inc) for w, _ in sizes],
+                "out": [run(ref, "ref_convert", *c) for c in cases]}
+    want = util.reference("oracle_pinning", f"line/{inc}/{outc}", theirs)
+    assert orc.orc_has_decoder(inc, outc) and want["has_decoder"]
+    assert [orc.orc_vc_get_linesize(w, inc) for w, _ in sizes] == want["linesize"]
+    for c, d in zip(cases, want["out"], strict=True):
+        assert run(orc, "orc_convert", *c) == d, (c[0], c[1], c[3])
 
 
-def test_v210_to_p010_vs_reference(orc, ref_cpu):
+def test_v210_to_p010_vs_reference(orc):
     for i, (w, h) in enumerate([(6, 2), (48, 4), (50, 6), (96, 5), (100, 7), (1920, 4), (7, 8), (13, 9)]):
         src = util.v210_noise(w, h, 50 + i)
         ls = ((w + 5) // 6 * 6) * 2 + 32
-        outs = []
-        for lib, fn in ((orc, "orc_v210_to_p010le"), (ref_cpu, "ref_v210_to_p010le")):
+
+        def run(lib, fn):
             y = np.full(ls * h, 0xAB, dtype=np.uint8)
             c = np.full(ls * ((h + 1) // 2), 0xCD, dtype=np.uint8)
             getattr(lib, fn)(w, h, y.ctypes.data, ls, c.ctypes.data, ls, src.ctypes.data)
-            outs.append((y, c))
-        assert np.array_equal(outs[0][0], outs[1][0]), (w, h)
-        assert np.array_equal(outs[0][1], outs[1][1]), (w, h)
+            return [util.digest(y), util.digest(c)]
+        assert run(orc, "orc_v210_to_p010le") == util.reference("oracle_pinning", f"v210_to_p010le/{w}x{h}",
+                                                                 lambda: run(util.ref_cpu(), "ref_v210_to_p010le")), (w, h)
 
 
 def test_v210_p010_identity(orc):

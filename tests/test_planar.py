@@ -1,5 +1,5 @@
 """Packed<->planar whole-buffer converters (SURVEY.md section 8 rows A10/A11): src/to_planar.c and src/from_planar.c of the reference.
-  * CPU: the restatement (oracle/planar_oracle.c) against the unmodified reference objects (oracle/_ref/libugref.so, when built);
+  * CPU: the restatement (oracle/planar_oracle.c) against the unmodified reference objects (oracle/_ref/libugref.so; their outputs recorded in tests/golden);
   * GPU: ugb200_<name> through the C ABI against the restatement, byte for byte, including the bytes that must stay untouched."""
 import numpy as np
 import pytest
@@ -28,16 +28,15 @@ def orc():
 
 @pytest.mark.parametrize("name,depth", pc.all_cases())
 def test_oracle_vs_reference(orc, name, depth):
-    ref = util.ref_cpu()
-    if ref is None:
-        pytest.skip("reference objects not built here (oracle/_ref)")
-    for i, (w, h) in enumerate(_sizes_for(name, True)):
-        for mode in (0, 1, 2):
-            for valid in (True, False):
-                c = pc.Case(name, w, h, seed=10 * i + mode, mode=mode, depth=depth, valid_bits=valid, shifts=((0, 8, 16), (16, 8, 0), (8, 16, 24))[mode])
-                a, b = c.run_cpu(orc, "orc_"), c.run_cpu(ref, "")
-                for k, (x, y) in enumerate(zip(a, b)):
-                    assert np.array_equal(x, y), (name, depth, w, h, mode, valid, k, np.flatnonzero(x != y)[:8])
+    sizes = _sizes_for(name, True)
+    cases = [[pc.Case(name, w, h, seed=10 * i + mode, mode=mode, depth=depth, valid_bits=valid, shifts=((0, 8, 16), (16, 8, 0), (8, 16, 24))[mode])
+              for mode in (0, 1, 2) for valid in (True, False)] for i, (w, h) in enumerate(sizes)]
+
+    def run(lib, prefix, size_cases):  # every output plane of every case of one size
+        return util.digest(*[o for c in size_cases for o in c.run_cpu(lib, prefix)])
+    want = util.reference("planar", f"{name}/{depth}", lambda: [run(util.ref_cpu(), "", cs) for cs in cases])
+    for (w, h), cs, d in zip(sizes, cases, want, strict=True):
+        assert run(orc, "orc_", cs) == d, (name, depth, w, h)
 
 
 @pytest.mark.gpu

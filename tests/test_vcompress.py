@@ -50,15 +50,18 @@ def test_module_lifecycle_without_frames(cfg):
 
 
 @pytest.mark.parametrize("cands", [(RGB, UYVY), (UYVY, RGB), (UYVY, RGB, RGBA), (RGBA, RGB), (UYVY,), (YUYV, UYVY)])
-def test_get_best_decoder_from_matches_reference(ref_cpu, cands):
+def test_get_best_decoder_from_matches_reference(cands):
     """where both sides have the converters, the selection (pixfmt_desc ranking 'dsc') must agree with the reference"""
     from ultragrid_b200 import compress
-    ref_cpu.ref_get_best_decoder_from.argtypes = [ctypes.c_int, ctypes.POINTER(ctypes.c_int), ctypes.c_int]
-    arr = (ctypes.c_int * len(cands))(*cands)
+    incs = (RGBA, UYVY, YUYV, V210, RGB, BGR, RG48)
+
+    def selections():  # per input codec: the reference's choice and the candidates it has a converter to
+        ref = util.ref_cpu()
+        ref.ref_get_best_decoder_from.argtypes = [ctypes.c_int, ctypes.POINTER(ctypes.c_int), ctypes.c_int]
+        arr = (ctypes.c_int * len(cands))(*cands)
+        return [[ref.ref_get_best_decoder_from(inc, arr, len(cands)), [c for c in cands if ref.ref_has_decoder(inc, c)]] for inc in incs]
     checked = 0
-    for inc in (RGBA, UYVY, YUYV, V210, RGB, BGR, RG48):
-        theirs = ref_cpu.ref_get_best_decoder_from(inc, arr, len(cands))
-        usable = [c for c in cands if ref_cpu.ref_has_decoder(inc, c)]
+    for inc, (theirs, usable) in zip(incs, util.reference("vcompress", "best_decoder/" + ",".join(map(str, cands)), selections), strict=True):
         if not all(compress.get_best_decoder_from(inc, [c]) == c for c in usable):
             continue  # the reference knows a converter that is not on the device yet: selection may legitimately differ
         assert compress.get_best_decoder_from(inc, cands) == theirs, (inc, cands)

@@ -3,7 +3,10 @@
 oracle/ is test infrastructure: it is loaded here (tests), by __graft_entry__.smoke() and by bench.py's
 cpu_baseline / --impl reference legs only.
 """
+import atexit
 import ctypes
+import hashlib
+import json
 import os
 import subprocess
 
@@ -11,6 +14,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
+GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
 
 _vp, _i, _l, _u = ctypes.c_void_p, ctypes.c_int, ctypes.c_long, ctypes.c_uint
 
@@ -158,6 +162,59 @@ def ref_gpu():
         getattr(L, n).argtypes = [_vp, _vp, _i, _i, _vp]
     L.cuda_yuv422_to_yuv444.argtypes = [_vp, _vp, _i, _vp]
     return L
+
+
+# ---- recorded results of the reference ----------------------------------------------------------------
+# The reference builds under oracle/_ref/ need the reference source tree, which a checkout of this project does not have.  What they
+# returned for the tests' inputs is stored in tests/golden/reference_<group>.json, so the comparisons run everywhere.  To record them again,
+# build oracle/_ref/ and run the tests with UGB200_RECORD_REFERENCE=<dir>: compute() then calls the reference and the results are written
+# to <dir>/reference_<group>.json.
+RECORD_DIR = os.environ.get("UGB200_RECORD_REFERENCE")
+_golden, _recorded = {}, {}
+
+
+def digest(*arrays):
+    """128-bit BLAKE2b of the bytes of the arrays (numpy or torch), in order: compares large outputs exactly without storing them"""
+    h = hashlib.blake2b(digest_size=16)
+    for a in arrays:
+        if hasattr(a, "cpu"):
+            a = a.cpu().numpy()
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def reference(group, key, compute):
+    """what the reference returned for one test input: compute() (JSON-able: ints, lists, dicts, digests) when recording, else the stored value"""
+    if RECORD_DIR:
+        value = json.loads(json.dumps(compute()))
+        _recorded.setdefault(group, {})[key] = value
+        return value
+    if group not in _golden:
+        with open(os.path.join(GOLDEN_DIR, f"reference_{group}.json")) as f:
+            _golden[group] = json.load(f)
+    assert key in _golden[group], f"no recorded reference result {group}:{key} (record it with UGB200_RECORD_REFERENCE)"
+    return _golden[group][key]
+
+
+def ref_color_coeffs(cs, depth):
+    """get_color_coeffs(cs, depth) of the unmodified src/color_space.c: the 14 ints it fills"""
+    def theirs():
+        out = (_i * 14)()
+        lib = ref_cpu()
+        lib.ref_get_color_coeffs(cs, depth, out)
+        return list(out)
+    return reference("color_space", f"{cs}/{depth}", theirs)
+
+
+@atexit.register
+def _write_recorded():
+    for group, table in _recorded.items():
+        path = os.path.join(RECORD_DIR, f"reference_{group}.json")
+        if os.path.exists(path):
+            with open(path) as f:
+                table = {**json.load(f), **table}
+        with open(path, "w") as f:  # one entry per line keeps diffs of the fixtures readable
+            f.write("{\n" + ",\n".join(f"{json.dumps(k)}: {json.dumps(table[k])}" for k in sorted(table)) + "\n}\n")
 
 
 def convert_cpu(lib, fn, in_c, out_c, src, width, height, dst_len=None, src_pitch=None, dst_pitch=None, shifts=(0, 8, 16),
